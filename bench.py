@@ -2,12 +2,13 @@
 """Benchmark of the `stride pbcorrect` hot path (seed discovery + FM extension + DP/MSA fallback) on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg3|cfg2|cfg3s|cfg1|mini] [--nodp]
+                    [--cli] [--extras] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over the WHOLE read set of the workload.  The default workload is BASELINE.json
 configs[2], the configuration its metric ("corrected Mbp/s at 1/2/4/8 B200") is quoted on: 12 Mb synthetic genome with
 injected repeats, 100x simulated CLR reads (mean 8 kb, 1.24 Gbp), `-c 100 -g 10`, the reference's default options
 (DP / multiple-alignment fallback on).  It fits one GPU.  `--workload cfg2` is configs[1] (4.6 Mb, 50x), also reported as a
-sub-result of the default line at N = 1.
+sub-result of the line at N = 1 with --extras.
 
 N > 1 (torchrun, one process per GPU): STRONG scaling of the product path.  Rank 0 simulates the reads and builds the index
 once; the flat index travels to the other GPUs as one blob over NCCL (NVLink), the reads through /dev/shm.  Every rank takes
@@ -20,7 +21,7 @@ lanes of its index (several batches in flight on separate streams).  No collecti
   parity  every read of the gathered e2e output is hashed (parity.py) and compared with the digests the UNMODIFIED reference
           produced (tests/golden/<workload>.read_sha.npz); `output_sha256` identifies the whole output and must be the same
           at every N
-  e2e_cli the shipped binary, `pbcorrect --gpus N`, on a FASTA file (reader -> N GPU workers -> in-order writer)
+  e2e_cli (--cli) the shipped binary, `pbcorrect --gpus N`, on a FASTA file (reader -> N GPU workers -> in-order writer)
 `--impl reference` times the reference's own multithreaded CPU implementation (oracle/_ref/stride pbcorrect -t <cores>)
 on a bounded sample of the same reads against the same index files, with the same options.
 """
@@ -42,6 +43,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the tree may be read-only: nothing of this run is cached there
 
 WORKLOADS = {
     # name: genome length, genome seed, coverage, mean read length, read seed, pbcorrect options
@@ -269,6 +271,42 @@ def run_threads(n_threads, n_items, fn):
 
 TIMING_KEYS = ("seed_ms", "extend_ms", "dp_ms", "walk_ms", "walk_launches", "dp_jobs", "dp_rows", "kernel_launches", "seed_pairs")
 
+# --dump-outputs: one seeded sample of the reads, drawn from the input lengths only, so that two builds dump the same reads;
+# counters of up to DUMP_READS reads and the corrected pieces of the first ~DUMP_PIECE_MBP input Mbp of the same permutation
+# (config 3: 100 k reads and ~4 M bases, ~30 MB of .npy files)
+DUMP_SEED = 20261020
+DUMP_READS = 100_000
+DUMP_PIECE_MBP = 4.0
+
+
+def dump_outputs(path, shard, batches, lengths):
+    """What the timed path returned for the reads of its last step (Batch.fetch: corrected pieces, their offsets, the first
+    piece of every read, the per-read counters), for the seeded sample above, as float64 .npy files (the bases as float32)."""
+    from longreadselfcorrect_b200 import api
+    perm = np.random.Generator(np.random.PCG64(DUMP_SEED)).permutation(lengths.size)
+    stat_ids = np.sort(perm[:DUMP_READS])
+    piece_ids = np.sort(perm[:int(np.searchsorted(np.cumsum(lengths[perm]), DUMP_PIECE_MBP * 1e6)) + 1])
+    stats = np.zeros(stat_ids.size, dtype=api.STATS_DTYPE)
+    n_pieces, piece_len, bases = [], [], []
+    for (f, _a, o), bt in zip(shard.batches, batches):
+        n = o.size - 1
+        out, poff, first, st = bt.fetch()
+        sel = stat_ids[(stat_ids >= f) & (stat_ids < f + n)]
+        stats[np.searchsorted(stat_ids, sel)] = st[sel - f]
+        for r in piece_ids[(piece_ids >= f) & (piece_ids < f + n)] - f:
+            p0, p1 = int(first[r]), int(first[r + 1])
+            n_pieces.append(p1 - p0)
+            piece_len.extend(int(poff[j + 1] - poff[j]) for j in range(p0, p1))
+            bases.append(out[int(poff[p0]):int(poff[p1])].copy())
+    os.makedirs(path, exist_ok=True)
+    arrays = {"stats_read_ids": stat_ids, "pieces_read_ids": piece_ids, "pieces_per_read": n_pieces, "piece_lengths": piece_len}
+    arrays.update({f"stats_{k}": stats[k] for k in api.STATS_DTYPE.names})
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
+    np.save(os.path.join(path, "pieces_bases.npy"), np.concatenate(bases).astype(np.float32) if bases else np.zeros(0, np.float32))
+    log(f"outputs of the last timed step: {stat_ids.size} reads' counters, {piece_ids.size} reads' pieces "
+        f"({sum(len(b) for b in bases)} bases) in {path}")
+
 
 def ours(args, wl, metric):
     import torch
@@ -278,6 +316,7 @@ def ours(args, wl, metric):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     cores = os.cpu_count() or 1
     assert torch.cuda.is_available(), "bench.py needs a CUDA device: the hot path has no CPU fallback"
+    assert not (args.dump_outputs and world > 1), "--dump-outputs needs one rank: the outputs of a step are spread over the ranks' shards"
     # --backend gloo: the same multi-rank code without NCCL (control traffic through gloo on CPU tensors), for boxes where the
     # ranks have to share one GPU (tests); PBSC_BENCH_SAME_DEVICE=1 puts every rank on GPU 0
     if os.environ.get("PBSC_BENCH_SAME_DEVICE") == "1":
@@ -426,6 +465,8 @@ def ours(args, wl, metric):
     ms_per_step = dev_ms / args.steps
     value = total_mbp / (ms_per_step / 1000)
     ph = {k: float(np.mean([p[k] for p in phases])) for k in TIMING_KEYS}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, shard, resident, lengths)
     if resident is not None:
         for bt in resident:
             bt.close()
@@ -761,12 +802,13 @@ def sub_results(args, local_rank):
     backward-search microbenchmark (config 5), each measured in a child process (fresh memory, bounded time)."""
     res = {}
     py = sys.executable
-    base = [py, os.path.abspath(__file__), "--no-extras", "--no-cpu-baseline", "--no-cli", "--e2e-steps", "1", "--steps", "3", "--warmup", "3"]
+    base = [py, os.path.abspath(__file__), "--no-cpu-baseline", "--steps", str(args.steps), "--warmup", str(args.warmup)]
+    env = dict(os.environ, PYTHONDONTWRITEBYTECODE="1")    # the children import modules of the tree, which must stay as build() left it
     for name, extra in (("cfg2_default_options", ["--workload", "cfg2"]), ("cfg2_nodp", ["--workload", "cfg2", "--nodp"])):
         if args.workload == "cfg2" and not args.nodp and name == "cfg2_default_options":
             continue
         try:
-            r = subprocess.run(base + extra, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=900)
+            r = subprocess.run(base + extra, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=900, env=env)
             j = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
             res[name] = {"value": j["value"], "unit": j["unit"], "ms_per_step": j["ms_per_step"], "e2e": j["e2e"], "config": j["config"]["workload"],
                          "parity_vs_reference": j.get("parity_vs_reference"), "roofline": j.get("roofline"), "phases_ms": j.get("phases_ms_rank0")}
@@ -775,13 +817,13 @@ def sub_results(args, local_rank):
     try:
         # index construction (SURVEY.md 8f-2): both strands of config 2 by pbsc_build_bwt; the reference's `stride index` on a 1 Mbp sample
         r = subprocess.run([py, os.path.join(ROOT, "tools", "index_bench.py"), "--json", "--workload", "cfg2", "--skip-torch", "--reference-mbp", "1"],
-                           stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=600)
+                           stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=600, env=env)
         res["index_build_cfg2"] = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
     except Exception as e:
         res["index_build_cfg2"] = {"error": str(e)[-200:]}
     try:
         r = subprocess.run([py, os.path.join(ROOT, "tools", "fm_microbench.py"), "--json", "--ks", "19,31", "--device", str(local_rank)],
-                           stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=600)
+                           stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=600, env=env)
         res["fm_microbench"] = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
     except Exception as e:
         res["fm_microbench"] = {"error": str(e)[-200:]}
@@ -800,13 +842,21 @@ def main():
     ap.add_argument("--cpu-sample-mbp", type=float, default=0.0, help="Mbp of reads for the CPU baseline (0 = auto)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-oracle-count", action="store_true", help="skip the instrumented-oracle and issued-sector counts of the roofline (profiles/algorithmic.json is used)")
-    ap.add_argument("--no-extras", dest="extras", action="store_false", help="skip the config 2 / --nodp / FM microbench sub-results")
-    ap.add_argument("--no-cli", dest="cli", action="store_false", help="skip the e2e_cli leg (the pbcorrect binary)")
-    ap.add_argument("--e2e-steps", type=int, default=2)
+    # asked for, not default: each adds minutes after the timed steps (a FASTA file of the whole read set through the binary, twice;
+    # three more workloads simulated and timed in child processes)
+    ap.add_argument("--extras", action="store_true", help="add the config 2 / --nodp / index build / FM microbench sub-results")
+    ap.add_argument("--cli", action="store_true", help="add the e2e_cli leg (the pbcorrect binary on a FASTA file)")
+    ap.add_argument("--e2e-steps", type=int, default=2, help="timed steps of the e2e leg (after one untimed pass)")
     ap.add_argument("--batch-mbp", type=float, default=256.0, help="largest batch of reads of one lane (Mbp)")
     ap.add_argument("--nodp", action="store_true", help="disable the DP/MSA fallback on both arms (seeds + FM extension only)")
     ap.add_argument("--backend", default="nccl", choices=["nccl", "gloo"], help="process-group backend for N > 1 (gloo: tests on a one-GPU box)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed for a fixed, seeded sample of the reads as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     wl = dict(WORKLOADS[args.workload])
     if args.nodp:
         wl["desc"] += " --nodp"

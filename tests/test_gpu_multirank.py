@@ -27,7 +27,7 @@ def _free_port():
 def _run_bench(world, extra=()):
     from longreadselfcorrect_b200 import api
     base = [sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "mini", "--gpus", str(world), "--steps", "1", "--warmup", "1", "--e2e-steps", "1",
-            "--no-extras", "--no-cpu-baseline", "--batch-mbp", "1.0"] + list(extra)
+            "--cli", "--no-cpu-baseline", "--batch-mbp", "1.0"] + list(extra)
     if world == 1:
         r = subprocess.run(base, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=420)
         assert r.returncode == 0, r.stderr[-1500:]
@@ -57,8 +57,8 @@ def _run_bench(world, extra=()):
     return json.loads([l for l in outs[0][0].splitlines() if l.startswith("{")][-1])
 
 
-def test_two_ranks_shard_the_product_path_and_reassemble_in_order():
-    one = _run_bench(1)
+def test_two_ranks_shard_the_product_path_and_reassemble_in_order(tmp_path):
+    one = _run_bench(1, ("--dump-outputs", str(tmp_path / "dump")))
     two = _run_bench(2)
     for j in (one, two):
         p = j["parity_vs_reference"]
@@ -68,3 +68,16 @@ def test_two_ranks_shard_the_product_path_and_reassemble_in_order():
     assert two["n_gpus"] == 2 and two["config"]["batches_per_rank"] >= 1
     # the shipped binary, driven by the same bench leg, writes the same records
     assert one["e2e_cli"]["output_sha256"] == one["parity_vs_reference"]["output_sha256"], one["e2e_cli"]
+    # --dump-outputs: the last timed step's counters of the sampled reads and the pieces of a sub-sample, consistent with each other
+    import numpy as np
+    d = {f[:-4]: np.load(tmp_path / "dump" / f) for f in os.listdir(tmp_path / "dump")}
+    ids, n = d["stats_read_ids"], one["config"]["reads"]
+    assert ids.dtype == np.float64 and ids.size == min(n, 100_000) and np.all(np.diff(ids) > 0)
+    assert all(d[k].shape == ids.shape for k in d if k.startswith("stats_"))
+    pids, npc = d["pieces_read_ids"], d["pieces_per_read"]
+    assert 0 < pids.size == npc.size and np.isin(pids, ids).all()
+    at = np.searchsorted(ids, pids)
+    assert np.array_equal(npc, d["stats_n_pieces"][at] * d["stats_merge"][at])      # a read that is not merged returns no piece
+    assert d["piece_lengths"].size == npc.sum() and d["pieces_bases"].dtype == np.float32
+    assert d["pieces_bases"].size == d["piece_lengths"].sum() and set(np.unique(d["pieces_bases"])) <= {65.0, 67.0, 71.0, 84.0}
+    assert sum(a.nbytes for a in d.values()) <= 64 << 20
