@@ -589,7 +589,7 @@ __global__ void __launch_bounds__(C::NT, 227 * 1024 / (C::SMEM + 1024))
 dp_align_thread_kernel(uint64_t n_rows, const uint32_t* __restrict__ keys, const uint32_t* __restrict__ order, DpRow* rows,
                        const DpJob* __restrict__ jobs, const WalkTask* __restrict__ tasks, uint8_t* mem, uint64_t mem0, uint32_t* arenas,
                        uint64_t arena_words, unsigned long long* counter, unsigned int* n_bad, const unsigned long long* __restrict__ n_eligible,
-                       unsigned long long min_rows, unsigned int* n_thread_rows, uint32_t* rarena)
+                       unsigned long long min_rows, unsigned int* n_thread_rows, uint32_t* rarena, int pair)
 {
     extern __shared__ uint32_t dpt_smem[];
     // One alignment per thread pays when there are enough of them to fill the machine: an alignment of L query bases is a
@@ -635,7 +635,7 @@ dp_align_thread_kernel(uint64_t n_rows, const uint32_t* __restrict__ keys, const
         const typename std::conditional<C::GREAD, DptSG, DptS<C>>::type S{Ss};
         const DptQ q{g.q};
         int bi, bj;
-        dpt::fill(g.qlen, g.mlen, g.origin, H, S, F, q, bi, bj);
+        dpt::fill(g.qlen, g.mlen, g.origin, H, S, F, q, bi, bj, pair != 0);
         if (bi <= 0) { atomicAdd(n_bad, 1u); R.pass = 0; }   // the reference would abort on its empty-cigar assert
         else
         {
@@ -784,6 +784,7 @@ DpStats& last_dp_stats() { static thread_local DpStats s; return s; }
 struct DptPass
 {
     bool on = false; uint64_t qmax = 0, arena_words = 0, min_rows = 0, read_words = 0; int blocks = 0;
+    int pair = 1;   // dpt::fill sweeps two columns at once where it can (PBSC_DPT_PAIR=0: one at a time)
     uint64_t flag_words() const { return on ? arena_words * (uint64_t)blocks : 0; }
 };
 template <class C>
@@ -814,7 +815,7 @@ static void dpt_pass_launch(const DptPass& g, cudaStream_t st, uint64_t nrows, D
     cub::DeviceRadixSort::SortPairs(sort_tmp, sort_bytes, keys, keys2, order, order2, (int)nrows, 0, DPT_KEY_BITS, st);
     const int tb = (int)std::min<uint64_t>((uint64_t)g.blocks, (nrows + C::NT - 1) / C::NT);
     dp_align_thread_kernel<C><<<tb, C::NT, C::SMEM, st>>>(nrows, keys2, order2, rows, jobs, tasks, mem, mem0, slabs, g.arena_words / (C::NT / 32), counter,
-                                                          cnt + 1, counter + 1, g.min_rows, cnt + 2, rarena);
+                                                          cnt + 1, counter + 1, g.min_rows, cnt + 2, rarena, g.pair);
 }
 
 int run_dp_fallback(pbsc_index* idx, const pbsc_params* p, DeviceBatch& b, void* tasks_v, uint64_t n_items, const uint32_t* list, uint8_t* outpool,
@@ -946,6 +947,8 @@ int run_dp_fallback(pbsc_index* idx, const pbsc_params* p, DeviceBatch& b, void*
         // warp-per-row kernel, which also serialises: a warp there fills 32 rows one after the other)
         pass_s.min_rows = 512; pass_l.min_rows = 2048; pass_h.min_rows = 2048;
         if (const char* e = getenv("PBSC_DPT_MIN_ROWS")) pass_s.min_rows = pass_l.min_rows = pass_h.min_rows = (uint64_t)std::max(0ll, atoll(e));
+        // PBSC_DPT_PAIR=0: the scalar fill, one column per sweep (for comparing the two; both give the same flags and scores)
+        if (const char* e = getenv("PBSC_DPT_PAIR")) pass_s.pair = pass_l.pair = pass_h.pair = atoi(e) != 0 ? 1 : 0;
         PBSC_CUDA(arena(idx, "dp.tkeys", max_rows, &tkeys));
         PBSC_CUDA(arena(idx, "dp.tkeys2", max_rows, &tkeys2));
         PBSC_CUDA(arena(idx, "dp.torder", max_rows, &torder));
