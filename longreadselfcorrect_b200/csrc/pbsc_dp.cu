@@ -485,22 +485,27 @@ dp_align_kernel(uint64_t n_rows, DpRow* rows, const DpJob* __restrict__ jobs, co
 // threads per block, three blocks per SM; longer ones up to 1024 bases with 64 threads per block (the 2-bit read in shared
 // memory is longer), four blocks per SM; up to 4000 bases (the 16-bit score limit) with one warp per block.  What is left
 // stays `pass == 2` for dp_align_kernel.
-template <int QMAX_, int NT_, bool GREAD_>
+template <int QMAX_, int NT_, bool GREAD_, bool RING_ = false>
 struct DptCfg
 {
     static constexpr int QMAX = QMAX_;                                          // longest query
     static constexpr int NT = NT_;                                              // threads per block
     static constexpr bool GREAD = GREAD_;                                       // the 2-bit read in global memory instead of shared
+    static constexpr bool RING = GREAD_ && RING_;                               // ... and the fill's window of it in a shared ring
     static constexpr int HWORDS = dpt::HSLOTS / 2;                              // 16-bit scores, two per word
     static constexpr int SWORDS = (dpt::max_len_bound(QMAX_) + 15) / 16 + 1;    // 2-bit read + one word of slack for bits()
-    static constexpr int SMEM = (HWORDS + (GREAD_ ? 0 : SWORDS)) * NT_ * 4;
+    static constexpr int RWORDS = 16;                                           // ring: words dpt::win_lo .. win_hi of a sweep
+    static constexpr int SMEM = (HWORDS + (GREAD_ ? (RING ? RWORDS : 0) : SWORDS)) * NT_ * 4;
 };
-// The previous column (512 B per alignment) has to be in shared memory; the read does not: for the longer queries it is kept in
-// global memory, word n of the 32 lanes of a warp side by side (coalesced, L1/L2 resident), which takes the resident warps per
-// SM from 8 to 12 (queries up to 1024 bases) and from 4 to 13 (up to 4000).
-using DptShort = DptCfg<256, 128, false>;   // 75 776 B per block: three blocks (12 warps) per SM
-using DptLong = DptCfg<1024, 64, true>;     // 32 768 B per block: six blocks (12 warps) per SM (51 456 B and 8 warps with the read in shared memory)
-using DptHuge = DptCfg<4000, 32, true>;     // 16 384 B per block: 13 blocks (13 warps) per SM; 8 * 4000 still fits 16 bits
+// The previous column (512 B per alignment) has to be in shared memory; the whole read does not: for the longer queries it is
+// kept in global memory, word n of the 32 lanes of a warp side by side (coalesced), which takes the resident warps per SM from
+// 8 to 12 (queries up to 1024 bases) and from 4 to 13 (up to 4000).  The fills of both passes read it from a ring of
+// 16 words per thread in shared memory that holds the window of the current sweep (DptSR): from global memory, most of its
+// reads were L2 hits on the dependency chain of the sweep.  The same ring in the 4000-base pass costs one block per SM (13 -> 12)
+// and still gains a little (profiles/r3_dpt_long_ab_cfg3s.txt).  The traceback reads the whole read from global memory.
+using DptShort = DptCfg<256, 128, false>;        // 75 776 B per block: three blocks (12 warps) per SM
+using DptLong = DptCfg<1024, 64, true, true>;    // 36 864 B per block: six blocks (12 warps) per SM (51 456 B and 8 warps with the whole read in shared memory)
+using DptHuge = DptCfg<4000, 32, true, true>;    // 18 432 B per block: 12 blocks (12 warps) per SM; 8 * 4000 still fits 16 bits
 constexpr uint32_t DPT_KEY_NONE = 0x3FFFu;
 constexpr int DPT_KEY_BITS = 14;
 
@@ -552,7 +557,19 @@ struct DptH   // previous column: 16-bit scores, slot j & 255, word (slot >> 1) 
     __device__ __forceinline__ bool pairs_ok(int j) const { return ((j >> 1) & (C::HWORDS - 1)) <= C::HWORDS - 5; }
     __device__ __forceinline__ uint32_t get2(int j, int u) const { return p[((j >> 1) & (C::HWORDS - 1)) * C::NT + u * C::NT]; }
     __device__ __forceinline__ void set2(int j, int u, uint32_t w) { p[((j >> 1) & (C::HWORDS - 1)) * C::NT + u * C::NT] = w; }
+#ifdef PBSC_STAGE_CLOCKS
+    long long clk_t = 0; unsigned long long clk[2] = {0, 0};   // dpt::clk_mark: time of the last mark, cycles per fill phase
+#endif
 };
+#ifdef PBSC_STAGE_CLOCKS
+template <class C>
+__device__ __forceinline__ void clk_mark(DptH<C>& H, int phase)
+{
+    const long long t = clock64();
+    H.clk[phase] += (unsigned long long)(t - H.clk_t);
+    H.clk_t = t;
+}
+#endif
 template <class C>
 struct DptS   // the retrieved read at 2 bits per base, 16 bases per word, in this thread's column of shared memory
 {
@@ -574,6 +591,36 @@ struct DptSG   // the same read in global memory: word n of this lane at p[n * 3
         return __funnelshift_r(w[0], w[32], 2 * (x & 15));
     }
 };
+template <class C>
+struct DptSR   // the fill's window of the read (dpt::win_lo .. win_hi of the sweep): word n in slot n & 15 of this thread's ring
+{
+    const uint32_t* g;   // the whole read in global memory, as DptSG
+    uint32_t* r;         // the ring: slot s at r[s * C::NT]
+    __device__ __forceinline__ int base(int x) const { return (int)((r[((x >> 4) & 15) * C::NT] >> (2 * (x & 15))) & 3u); }
+    __device__ __forceinline__ uint32_t bits(int x) const
+    {
+        return __funnelshift_r(r[((x >> 4) & 15) * C::NT], r[(((x >> 4) + 1) & 15) * C::NT], 2 * (x & 15));
+    }
+};
+struct DptRingWord { uint32_t w; int n; };   // word n of the read for the ring, n < 0: none
+// the fill's hooks (pbsc_dp_thread.cuh): load the word the sweep from inext adds to the window, store it after the sweep from i
+template <class C>
+__device__ __forceinline__ DptRingWord win_fetch(const DptSR<C>& S, int mlen, int origin, int i, int inext)
+{
+    const int n = dpt::win_hi(inext, mlen, origin);
+    DptRingWord x{0u, -1};
+    if (n >= 0 && n > dpt::win_hi(i, mlen, origin)) { x.w = S.g[(size_t)n * 32]; x.n = n; }
+    return x;
+}
+template <class C>
+__device__ __forceinline__ void win_store(const DptSR<C>& S, const DptRingWord& x) { if (x.n >= 0) S.r[(x.n & 15) * C::NT] = x.w; }
+template <class C>
+__device__ __forceinline__ auto dpt_fill_read(const uint32_t* s, uint32_t* r)
+{
+    if constexpr (C::RING) return DptSR<C>{s, r};
+    else if constexpr (C::GREAD) return DptSG{s};
+    else return DptS<C>{s};
+}
 struct DptF   // flag words of this lane: word n of the lane at arena[n * 32 + lane] (a warp's stores coalesce)
 {
     uint32_t* p;
@@ -582,6 +629,14 @@ struct DptF   // flag words of this lane: word n of the lane at arena[n * 32 + l
 };
 struct DptQ { const uint8_t* q; __device__ __forceinline__ int operator()(int x) const { return (int)q[x]; } };
 struct DptOps { uint8_t* ops; __device__ __forceinline__ void put(int n, int op) { ops[n] = (uint8_t)op; } };
+
+// -DPBSC_STAGE_CLOCKS (measurement build, not for timing runs): per pass (0: <= 256, 1: <= 1024, 2: <= 4000), the clock64()
+// cycles of every lane in row setup, fill column ends (single steps and one-column fills), paired blocks, traceback, filters
+// and row store; then rows, computed cells and traceback steps.  Printed as "[pbsc dpt clocks]" by run_dp_fallback.
+#ifdef PBSC_STAGE_CLOCKS
+constexpr int DPT_CLK_N = 8;
+__device__ unsigned long long g_dpt_clk[3][DPT_CLK_N];
+#endif
 
 // arena_words: flag words of one warp's 32 rows = 32 * (longest query of this pass) * WMAX
 template <class C>
@@ -604,7 +659,15 @@ dp_align_thread_kernel(uint64_t n_rows, const uint32_t* __restrict__ keys, const
     // the read's words: this thread's column of shared memory, or this lane's column of the warp's slab in global memory
     uint32_t* Ss = C::GREAD ? rarena + warp * (uint64_t)(C::SWORDS * 32) + lane : dpt_smem + C::HWORDS * C::NT + threadIdx.x;
     constexpr int SSTRIDE = C::GREAD ? 32 : C::NT;
+    uint32_t* Rs = dpt_smem + C::HWORDS * C::NT + threadIdx.x;   // the ring of the read's words (C::RING)
     DptF F{arenas + warp * arena_words + lane};
+#ifdef PBSC_STAGE_CLOCKS
+    unsigned long long clk[DPT_CLK_N] = {0, 0, 0, 0, 0, 0, 0, 0};
+    long long clk_t = clock64();
+#define DPT_CLK(i) do { const long long t_ = clock64(); clk[i] += (unsigned long long)(t_ - clk_t); clk_t = t_; } while (0)
+#else
+#define DPT_CLK(i) do { } while (0)
+#endif
     for (;;)
     {
         unsigned long long base = 0;
@@ -620,28 +683,48 @@ dp_align_thread_kernel(uint64_t n_rows, const uint32_t* __restrict__ keys, const
         const DpJob J = jobs[R.job];
         RowGeom g;
         row_geometry(R, J, mem, mem0, g);
-        // the read at 2 bits per base, the column at zero
+        // the read at 2 bits per base (and the first sweep's window of it in the ring), the column at zero
+        const int rlo = dpt::win_lo(1, g.origin), rhi = dpt::win_hi(1, g.mlen, g.origin);
         for (int x = 0; x < g.mlen; x += 16)
         {
             uint32_t w = 0;
             const int m = min(16, g.mlen - x);
             for (int y = 0; y < m; y++) w |= (uint32_t)g.s2[x + y] << (2 * y);
             Ss[(x >> 4) * SSTRIDE] = w;
+            if (C::RING && (x >> 4) >= rlo && (x >> 4) <= rhi) Rs[((x >> 4) & 15) * C::NT] = w;
         }
         Ss[((g.mlen + 15) >> 4) * SSTRIDE] = 0u;
+        if (C::RING && ((g.mlen + 15) >> 4) <= rhi) Rs[(((g.mlen + 15) >> 4) & 15) * C::NT] = 0u;
         #pragma unroll 8
         for (int x = 0; x < C::HWORDS; x++) Hs[x * C::NT] = 0u;
         DptH<C> H{Hs};
-        const typename std::conditional<C::GREAD, DptSG, DptS<C>>::type S{Ss};
+        const auto SF = dpt_fill_read<C>(Ss, Rs);                                 // the fill's read
+        const typename std::conditional<C::GREAD, DptSG, DptS<C>>::type S{Ss};   // the traceback's
         const DptQ q{g.q};
         int bi, bj;
-        dpt::fill(g.qlen, g.mlen, g.origin, H, S, F, q, bi, bj, pair != 0);
+        DPT_CLK(0);
+#ifdef PBSC_STAGE_CLOCKS
+        H.clk_t = clk_t;
+#endif
+        dpt::fill(g.qlen, g.mlen, g.origin, H, SF, F, q, bi, bj, pair != 0);
+#ifdef PBSC_STAGE_CLOCKS
+        clk[1] += H.clk[dpt::CLK_ENDS]; clk[2] += H.clk[dpt::CLK_BLOCKS];
+        clk_t = H.clk_t;
+        DPT_CLK(1);   // the last column's scan for the traceback start
+        clk[5]++;
+        for (int i = 1; i <= g.qlen; i++) clk[6] += (unsigned long long)max(0, min(g.origin + i + dpt::BW, g.mlen + 1) - max(g.origin + i, 1));
+        clk_t = clock64();   // the count above is no phase
+#endif
         if (bi <= 0) { atomicAdd(n_bad, 1u); R.pass = 0; }   // the reference would abort on its empty-cigar assert
         else
         {
             DptOps ops{g.ops};
             int n, ed, i0, j0;
             dpt::traceback(g.qlen, g.mlen, g.origin, S, F, q, bi, bj, ops, n, ed, i0, j0);
+            DPT_CLK(3);
+#ifdef PBSC_STAGE_CLOCKS
+            clk[7] += (unsigned long long)n;
+#endif
             const WalkTask& tk = tasks[J.task];
             // identity = 0.65 (+0.05 above 50, +0.05 above 100), min_overlap = path.length()/10
             // (PacBioSelfCorrectionProcess.cpp:225-235)
@@ -656,7 +739,13 @@ dp_align_thread_kernel(uint64_t n_rows, const uint32_t* __restrict__ keys, const
             R.pass = (passOverlap && passIdentity) ? 1u : 0u;
         }
         rows[ri] = R;
+        DPT_CLK(4);
     }
+#ifdef PBSC_STAGE_CLOCKS
+    constexpr int pass = C::QMAX <= 256 ? 0 : C::QMAX <= 1024 ? 1 : 2;
+    for (int x = 0; x < DPT_CLK_N; x++) atomicAdd(&g_dpt_clk[pass][x], clk[x]);
+#endif
+#undef DPT_CLK
 }
 
 // ---- stage 3: thread per job: multiple alignment on per-column counts, consensus ---------------------------------------
@@ -1078,6 +1167,25 @@ int run_dp_fallback(pbsc_index* idx, const pbsc_params* p, DeviceBatch& b, void*
     PBSC_CUDA(cudaStreamSynchronize(st));
     S.bad += hcnt[1];
     S.thread_rows += hcnt[2];
+#ifdef PBSC_STAGE_CLOCKS
+    {
+        unsigned long long h[3][DPT_CLK_N], z[3][DPT_CLK_N] = {};
+        cudaMemcpyFromSymbol(h, g_dpt_clk, sizeof h);
+        cudaMemcpyToSymbol(g_dpt_clk, z, sizeof z);
+        static const char* pass_names[3] = {"256", "1024", "4000"};
+        static const char* names[5] = {"setup", "ends", "blocks", "traceback", "filters+store"};
+        for (int x = 0; x < 3; x++)
+        {
+            if (!h[x][5]) continue;
+            unsigned long long tot = 0;
+            for (int i = 0; i < 5; i++) tot += h[x][i];
+            fprintf(stderr, "[pbsc dpt clocks] pass %-4s rows %llu cells %llu traceback-steps %llu lane-cycles %llu (%.1f per cell);", pass_names[x],
+                    h[x][5], h[x][6], h[x][7], tot, h[x][6] ? (double)tot / (double)h[x][6] : 0.0);
+            for (int i = 0; i < 5; i++) fprintf(stderr, " %s %.1f %%;", names[i], tot ? 100.0 * (double)h[x][i] / (double)tot : 0.0);
+            fprintf(stderr, "\n");
+        }
+    }
+#endif
     PBSC_OCC_TAKE(3, st);
     float ms = 0;
     cudaEventElapsedTime(&ms, ev[0], ev[1]);

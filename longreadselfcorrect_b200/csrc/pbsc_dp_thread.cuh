@@ -129,6 +129,11 @@ PBSC_DPT_HD uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel)
 #endif
 }
 
+// Phase hook of the fill: clk_mark(H, p) charges the time since the previous mark to phase p.  A no-op for every accessor
+// except the one of the kernel's -DPBSC_STAGE_CLOCKS measurement build (pbsc_dp.cu), which overloads it.
+constexpr int CLK_ENDS = 0, CLK_BLOCKS = 1;   // single steps and one-column fills; paired blocks
+template <class HS> PBSC_DPT_HD void clk_mark(HS&, int) {}
+
 // running state of the fill across columns
 struct FillBest { int rowVal = 0, rowI = 0; bool anyRow = false; };
 PBSC_DPT_HD void note_last_row(FillBest& b, int v, int i)
@@ -237,6 +242,7 @@ PBSC_DPT_HD void fill_col(int i, int mlen, int origin, int wbase, HS& H, const S
         }
         if (kin) F.put(widx, w << (3 * (CPW - kin)));
         if (last == nRows - 1) note_last_row(best, v, i);
+        clk_mark(H, CLK_ENDS);
     }
 }
 
@@ -354,6 +360,7 @@ PBSC_DPT_HD void fill_pair(int i, int mlen, int origin, int wbase, HS& H, const 
     #pragma unroll 1
 #endif
     for (; j < jw; j++) step(j);
+    clk_mark(H, CLK_ENDS);
     // here, at every block: A has no pending flags, B has nine (rows j - 10 .. j - 2)
 #if defined(__CUDA_ARCH__)
     #pragma unroll 1
@@ -413,6 +420,7 @@ PBSC_DPT_HD void fill_pair(int i, int mlen, int origin, int wbase, HS& H, const 
         hA = lo16(D); a2 = hi16(D); a1 = lo16(V); b1 = hi16(V);
 #endif
         H.set(j - 2, b1);   // the last block left B(j - 2) for the next one
+        clk_mark(H, CLK_BLOCKS);
     }
     // the rest reads rows j - 1 .. lA (bases j - 2 .. lA - 1 <= j + 8) and B's last row lB <= lA + 1 (base lB - 1 <= lA)
     sx0 = j - 2;
@@ -426,7 +434,27 @@ PBSC_DPT_HD void fill_pair(int i, int mlen, int origin, int wbase, HS& H, const 
     if (kB) F.put(xB, wB << (3 * (CPW - kB)));
     if (lA == nRows - 1) note_last_row(best, vAl, i);
     if (lB == nRows - 1) note_last_row(best, vBl, i + 1);
+    clk_mark(H, CLK_ENDS);
 }
+
+// Read window.  A sweep from column i (fill_col, or fill_pair of i and i + 1) reads the read from base origin + i - 1 on, and
+// S.bits at origin + i + 200 at most, which takes that base's word and the next one; with 16 bases per word, those are words
+// win_lo(i) .. win_hi(i), at most 15, clipped to the read and the zero word after it.  win_hi grows by at most one word from
+// a sweep to the next (two columns on), and win_hi(i + 2) <= win_lo(i) + 14: the ring slot of the word it adds holds a word at
+// least two below win_lo(i), which the sweep before does not read.  So an accessor that keeps only a ring of 16 words of the
+// read (the kernel's global-read passes, pbsc_dp.cu) needs one load per sweep: fill() calls win_fetch(S, mlen, origin, i, inext) before the sweep from i and win_store(S, what it returned) after
+// it, and the next sweep from inext finds its words in the ring.  For an accessor that holds the whole read both do nothing.
+PBSC_DPT_HD int win_lo(int i, int origin) { return imax(origin + i - 1, 0) >> 4; }
+PBSC_DPT_HD int win_hi(int i, int mlen, int origin) { return imin(((origin + i + BW - 1) >> 4) + 1, (mlen + 15) >> 4); }
+template <class SS> PBSC_DPT_HD int win_fetch(const SS&, int /*mlen*/, int /*origin*/, int /*i*/, int /*inext*/) { return 0; }
+template <class SS, class T> PBSC_DPT_HD void win_store(const SS&, const T&) {}
+
+// the two query bases a sweep from column i reads, q(i - 1) and q(i), loaded before it
+struct QCols
+{
+    int i0, c0, c1;
+    PBSC_DPT_HD int operator()(int x) const { return x == i0 ? c0 : c1; }
+};
 
 // Whole fill: columns 1..qlen, in pairs where pairable() allows (pair = false: one column at a time throughout); (bi, bj) =
 // start of the traceback, bi = 0 when there is none.
@@ -437,21 +465,25 @@ PBSC_DPT_HD void fill(int qlen, int mlen, int origin, HS& H, const SS& S, FS& F,
     const int W = words_per_col(mlen);
     FillBest best;
     int i = 1, wbase = 0;
+    // the query bases of a sweep (columns i, i + 1) and the read word the next sweep adds to a window accessor are loaded one
+    // sweep ahead, so that no sweep starts on a load
+    int c0 = q(0), c1 = qlen > 1 ? q(1) : 0;
+    bool pr = pair && 1 < qlen && pairable(1, mlen, origin);
 #if defined(__CUDA_ARCH__)
     #pragma unroll 1
 #endif
     while (i <= qlen)
     {
-        if (pair && i < qlen && pairable(i, mlen, origin))
-        {
-            fill_pair(i, mlen, origin, wbase, H, S, F, q, best);
-            i += 2; wbase += 2 * W;
-        }
-        else
-        {
-            fill_col(i, mlen, origin, wbase, H, S, F, q, best);
-            i++; wbase += W;
-        }
+        const int inext = i + (pr ? 2 : 1);
+        const auto wn = win_fetch(S, mlen, origin, i, inext);
+        const int n0 = inext <= qlen ? q(inext - 1) : 0, n1 = inext < qlen ? q(inext) : 0;
+        const QCols qc{i - 1, c0, c1};
+        if (pr) fill_pair(i, mlen, origin, wbase, H, S, F, qc, best);
+        else fill_col(i, mlen, origin, wbase, H, S, F, qc, best);
+        win_store(S, wn);
+        wbase += (inext - i) * W;
+        i = inext; c0 = n0; c1 = n1;
+        pr = pair && i < qlen && pairable(i, mlen, origin);
     }
     const int bestRowVal = best.rowVal, bestRowI = best.rowI;
     const bool anyRow = best.anyRow;
