@@ -558,7 +558,7 @@ struct DptH   // previous column: 16-bit scores, slot j & 255, word (slot >> 1) 
     __device__ __forceinline__ uint32_t get2(int j, int u) const { return p[((j >> 1) & (C::HWORDS - 1)) * C::NT + u * C::NT]; }
     __device__ __forceinline__ void set2(int j, int u, uint32_t w) { p[((j >> 1) & (C::HWORDS - 1)) * C::NT + u * C::NT] = w; }
 #ifdef PBSC_STAGE_CLOCKS
-    long long clk_t = 0; unsigned long long clk[2] = {0, 0};   // dpt::clk_mark: time of the last mark, cycles per fill phase
+    long long clk_t = 0; unsigned long long clk[3] = {0, 0, 0}, cells[3] = {0, 0, 0};   // dpt::clk_mark: time of the last mark, cycles per fill phase; dpt::clk_cells: cells per fill path
 #endif
 };
 #ifdef PBSC_STAGE_CLOCKS
@@ -569,6 +569,8 @@ __device__ __forceinline__ void clk_mark(DptH<C>& H, int phase)
     H.clk[phase] += (unsigned long long)(t - H.clk_t);
     H.clk_t = t;
 }
+template <class C>
+__device__ __forceinline__ void clk_cells(DptH<C>& H, int path, int n) { H.cells[path] += (unsigned long long)n; }
 #endif
 template <class C>
 struct DptS   // the retrieved read at 2 bits per base, 16 bases per word, in this thread's column of shared memory
@@ -631,10 +633,11 @@ struct DptQ { const uint8_t* q; __device__ __forceinline__ int operator()(int x)
 struct DptOps { uint8_t* ops; __device__ __forceinline__ void put(int n, int op) { ops[n] = (uint8_t)op; } };
 
 // -DPBSC_STAGE_CLOCKS (measurement build, not for timing runs): per pass (0: <= 256, 1: <= 1024, 2: <= 4000), the clock64()
-// cycles of every lane in row setup, fill column ends (single steps and one-column fills), paired blocks, traceback, filters
-// and row store; then rows, computed cells and traceback steps.  Printed as "[pbsc dpt clocks]" by run_dp_fallback.
+// cycles of every lane in row setup, one-column fills (with the last column's scan), masked paired blocks, unmasked paired
+// blocks, traceback, filters and row store; then rows, computed cells and traceback steps; then the cells computed by
+// unmasked blocks, masked blocks and one-column fills.  Printed as "[pbsc dpt clocks]" by run_dp_fallback.
 #ifdef PBSC_STAGE_CLOCKS
-constexpr int DPT_CLK_N = 8;
+constexpr int DPT_CLK_N = 12;
 __device__ unsigned long long g_dpt_clk[3][DPT_CLK_N];
 #endif
 
@@ -662,7 +665,7 @@ dp_align_thread_kernel(uint64_t n_rows, const uint32_t* __restrict__ keys, const
     uint32_t* Rs = dpt_smem + C::HWORDS * C::NT + threadIdx.x;   // the ring of the read's words (C::RING)
     DptF F{arenas + warp * arena_words + lane};
 #ifdef PBSC_STAGE_CLOCKS
-    unsigned long long clk[DPT_CLK_N] = {0, 0, 0, 0, 0, 0, 0, 0};
+    unsigned long long clk[DPT_CLK_N] = {};
     long long clk_t = clock64();
 #define DPT_CLK(i) do { const long long t_ = clock64(); clk[i] += (unsigned long long)(t_ - clk_t); clk_t = t_; } while (0)
 #else
@@ -708,11 +711,12 @@ dp_align_thread_kernel(uint64_t n_rows, const uint32_t* __restrict__ keys, const
 #endif
         dpt::fill(g.qlen, g.mlen, g.origin, H, SF, F, q, bi, bj, pair != 0);
 #ifdef PBSC_STAGE_CLOCKS
-        clk[1] += H.clk[dpt::CLK_ENDS]; clk[2] += H.clk[dpt::CLK_BLOCKS];
+        clk[1] += H.clk[dpt::CLK_COLS]; clk[2] += H.clk[dpt::CLK_MASKED]; clk[3] += H.clk[dpt::CLK_BLOCKS];
+        clk[9] += H.cells[dpt::CLK_BLOCKS]; clk[10] += H.cells[dpt::CLK_MASKED]; clk[11] += H.cells[dpt::CLK_COLS];
         clk_t = H.clk_t;
         DPT_CLK(1);   // the last column's scan for the traceback start
-        clk[5]++;
-        for (int i = 1; i <= g.qlen; i++) clk[6] += (unsigned long long)max(0, min(g.origin + i + dpt::BW, g.mlen + 1) - max(g.origin + i, 1));
+        clk[6]++;
+        for (int i = 1; i <= g.qlen; i++) clk[7] += (unsigned long long)max(0, min(g.origin + i + dpt::BW, g.mlen + 1) - max(g.origin + i, 1));
         clk_t = clock64();   // the count above is no phase
 #endif
         if (bi <= 0) { atomicAdd(n_bad, 1u); R.pass = 0; }   // the reference would abort on its empty-cigar assert
@@ -721,9 +725,9 @@ dp_align_thread_kernel(uint64_t n_rows, const uint32_t* __restrict__ keys, const
             DptOps ops{g.ops};
             int n, ed, i0, j0;
             dpt::traceback(g.qlen, g.mlen, g.origin, S, F, q, bi, bj, ops, n, ed, i0, j0);
-            DPT_CLK(3);
+            DPT_CLK(4);
 #ifdef PBSC_STAGE_CLOCKS
-            clk[7] += (unsigned long long)n;
+            clk[8] += (unsigned long long)n;
 #endif
             const WalkTask& tk = tasks[J.task];
             // identity = 0.65 (+0.05 above 50, +0.05 above 100), min_overlap = path.length()/10
@@ -739,7 +743,7 @@ dp_align_thread_kernel(uint64_t n_rows, const uint32_t* __restrict__ keys, const
             R.pass = (passOverlap && passIdentity) ? 1u : 0u;
         }
         rows[ri] = R;
-        DPT_CLK(4);
+        DPT_CLK(5);
     }
 #ifdef PBSC_STAGE_CLOCKS
     constexpr int pass = C::QMAX <= 256 ? 0 : C::QMAX <= 1024 ? 1 : 2;
@@ -1173,16 +1177,16 @@ int run_dp_fallback(pbsc_index* idx, const pbsc_params* p, DeviceBatch& b, void*
         cudaMemcpyFromSymbol(h, g_dpt_clk, sizeof h);
         cudaMemcpyToSymbol(g_dpt_clk, z, sizeof z);
         static const char* pass_names[3] = {"256", "1024", "4000"};
-        static const char* names[5] = {"setup", "ends", "blocks", "traceback", "filters+store"};
+        static const char* names[6] = {"setup", "columns", "masked-blocks", "blocks", "traceback", "filters+store"};
         for (int x = 0; x < 3; x++)
         {
-            if (!h[x][5]) continue;
+            if (!h[x][6]) continue;
             unsigned long long tot = 0;
-            for (int i = 0; i < 5; i++) tot += h[x][i];
+            for (int i = 0; i < 6; i++) tot += h[x][i];
             fprintf(stderr, "[pbsc dpt clocks] pass %-4s rows %llu cells %llu traceback-steps %llu lane-cycles %llu (%.1f per cell);", pass_names[x],
-                    h[x][5], h[x][6], h[x][7], tot, h[x][6] ? (double)tot / (double)h[x][6] : 0.0);
-            for (int i = 0; i < 5; i++) fprintf(stderr, " %s %.1f %%;", names[i], tot ? 100.0 * (double)h[x][i] / (double)tot : 0.0);
-            fprintf(stderr, "\n");
+                    h[x][6], h[x][7], h[x][8], tot, h[x][7] ? (double)tot / (double)h[x][7] : 0.0);
+            for (int i = 0; i < 6; i++) fprintf(stderr, " %s %.1f %%;", names[i], tot ? 100.0 * (double)h[x][i] / (double)tot : 0.0);
+            fprintf(stderr, " cells in blocks %llu, masked blocks %llu, columns %llu;\n", h[x][9], h[x][10], h[x][11]);
         }
     }
 #endif

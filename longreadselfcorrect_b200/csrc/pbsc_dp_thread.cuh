@@ -10,7 +10,8 @@
 // The code below is plain scalar C++ over four small accessor types, so that tests/cpp/test_dp_thread.cpp can compile the
 // very same fill/traceback with g++ and compare it with the oracle; the kernel instantiates it with shared-memory and
 // interleaved-global accessors (pbsc_dp.cu).  Where two neighbouring columns allow it, the fill sweeps both at once with two
-// 16-bit scores per register (fill_pair); tests/cpp/test_dp_pair.cpp checks that against the one-column fill (fill_col).
+// 16-bit scores per register (fill_pair); tests/cpp/test_dp_pair.cpp and test_dp_pair_masked.cpp check that against the
+// one-column fill (fill_col).
 //
 // Rules reproduced (all relative to the reference's band table, band row r = j - (origin + i), 0 <= r <= 200):
 //   * the table is zero-initialised and column 0 / row 0 are never written: they read as 0;
@@ -74,9 +75,9 @@ PBSC_DPT_HD int words_per_col(int mlen) { return (imin(BW, mlen) + 1 + CPW - 1) 
 // ---- two 16-bit scores in one 32-bit word: the low half belongs to column i, the high half to column i + 1 ----------------
 // Device: the sm_100 SIMD instructions (VIADD.16x2, VIMNMX3.S16x2, VIADDMNMX.S16x2, PRMT).  Host: the same lane arithmetic,
 // which aborts if a lane leaves the int16 range, so the host tests catch a packed score that would wrap.
-#if !defined(__CUDA_ARCH__)
 PBSC_DPT_HD int lo16(uint32_t x) { return (int)(int16_t)(x & 0xFFFFu); }
 PBSC_DPT_HD int hi16(uint32_t x) { return (int)(int16_t)(x >> 16); }
+#if !defined(__CUDA_ARCH__)
 PBSC_DPT_HD uint32_t pk16(int lo, int hi)
 {
     if (lo < -32768 || lo > 32767 || hi < -32768 || hi > 32767) { printf("packed 16-bit lane overflow\n"); abort(); }
@@ -116,6 +117,23 @@ PBSC_DPT_HD uint32_t v2addmax(uint32_t a, uint32_t b, uint32_t c)
     return pk16(imax(lo16(a) + lo16(b), lo16(c)), imax(hi16(a) + hi16(b), hi16(c)));
 #endif
 }
+// min(a + b, c) per half
+PBSC_DPT_HD uint32_t v2addmin(uint32_t a, uint32_t b, uint32_t c)
+{
+#if defined(__CUDA_ARCH__)
+    return __viaddmin_s16x2(a, b, c);
+#else
+    return pk16(imin(lo16(a) + lo16(b), lo16(c)), imin(hi16(a) + hi16(b), hi16(c)));
+#endif
+}
+PBSC_DPT_HD uint32_t v2max(uint32_t a, uint32_t b)
+{
+#if defined(__CUDA_ARCH__)
+    return __vmaxs2(a, b);
+#else
+    return pk16(imax(lo16(a), lo16(b)), imax(hi16(a), hi16(b)));
+#endif
+}
 // bytes of (b:a) picked by the four nibbles of sel (__byte_perm without the sign-replicate mode)
 PBSC_DPT_HD uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel)
 {
@@ -129,10 +147,27 @@ PBSC_DPT_HD uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel)
 #endif
 }
 
-// Phase hook of the fill: clk_mark(H, p) charges the time since the previous mark to phase p.  A no-op for every accessor
-// except the one of the kernel's -DPBSC_STAGE_CLOCKS measurement build (pbsc_dp.cu), which overloads it.
-constexpr int CLK_ENDS = 0, CLK_BLOCKS = 1;   // single steps and one-column fills; paired blocks
+// the bits of b where m is set, those of a elsewhere (one LOP3); m selects whole 16-bit halves here
+PBSC_DPT_HD uint32_t sel16(uint32_t a, uint32_t b, uint32_t m) { return (a & ~m) | (b & m); }
+PBSC_DPT_HD int popc(uint32_t x)
+{
+#if defined(__CUDA_ARCH__)
+    return __popc(x);
+#else
+    return __builtin_popcount(x);
+#endif
+}
+
+// Phase hooks of the fill: clk_mark(H, p) charges the time since the previous mark to phase p, clk_cells(H, p, n) counts n
+// computed cells for the path p.  No-ops for every accessor except the one of the kernel's -DPBSC_STAGE_CLOCKS measurement
+// build (pbsc_dp.cu), which overloads them.
+constexpr int CLK_COLS = 0, CLK_MASKED = 1, CLK_BLOCKS = 2;   // one-column fills; masked paired blocks; unmasked paired blocks
 template <class HS> PBSC_DPT_HD void clk_mark(HS&, int) {}
+template <class HS> PBSC_DPT_HD void clk_cells(HS&, int, int) {}
+// Hook of the paired fill: pair_sweep(H, fB, lB) before a sweep of fill_pair, whose second column computes rows fB .. lB, and
+// pair_sweep(H, 1, 0) after it.  A no-op except for the accessor of the host test tests/cpp/test_dp_pair_masked.cpp, which
+// checks the sweep's stores against those rows.
+template <class HS> PBSC_DPT_HD void pair_sweep(HS&, int, int) {}
 
 // running state of the fill across columns
 struct FillBest { int rowVal = 0, rowI = 0; bool anyRow = false; };
@@ -242,7 +277,8 @@ PBSC_DPT_HD void fill_col(int i, int mlen, int origin, int wbase, HS& H, const S
         }
         if (kin) F.put(widx, w << (3 * (CPW - kin)));
         if (last == nRows - 1) note_last_row(best, v, i);
-        clk_mark(H, CLK_ENDS);
+        clk_cells(H, CLK_COLS, last - first + 1);
+        clk_mark(H, CLK_COLS);
     }
 }
 
@@ -262,18 +298,31 @@ PBSC_DPT_HD bool pairable(int i, int mlen, int origin)
 // of column i - 1 in H, which A read last at step j - 1, so after the sweep H holds column i + 1 (rows of column i are
 // never stored: nothing reads them).  Each column keeps its own flag words, exactly as fill_col writes them.
 //
-// The packed block: ten steps with every cell of both columns a middle cell, one 32-bit register per quantity, A in the low
-// half and B in the high half:
+// The sweep is a run of ten-step blocks from A's row j0 = fA & ~1, where the flag ordinals of both columns start, until B's
+// last row lB is computed.  A block from row j writes A's flag word of rows j .. j + 9 and completes B's of rows j - 10 ..
+// j - 1.  One 32-bit register per quantity, A in the low half and B in the high half:
 //   up = the result of the step before; left = (column i - 1 at row j, A(j - 1)), one PRMT from H's pair word; diagonal =
 //   the left of the step before; x = max(d + 1, left, up) with d + 1 = diagonal + (2 or -7), and the "equals" flags from
 //   max(candidate + 2 - x, 1), which is 2 or 1 per half.  Five pair stores of B per block (rows j - 2 .. j + 7; B(j + 8) is
 //   stored after the last block).  Every pair is addressed on its own, so a block may wrap around H's circular array: rows of
 //   a warp's alignments reach the wrap at different blocks, and a branch there would make the warp run both paths.
-// The first ten rows of A and whatever follows the last block run one step at a time in 32-bit arithmetic (step below), with
-// the same rules as fill_col.
+// A block whose twenty cells are all middle cells of their columns runs as just described.  The first block and the last one
+// or two (the masked blocks) apply fill_col's rules per half with selects, from bit masks of the block's steps computed once
+// per block:
+//   * first cell (row fA, fB): "up" is the sentinel in the max; the flags compare it with row 0 (0) when the band top is
+//     above the matrix, else never;
+//   * last cell (row lA, lB) when it is not also the first, or when it is band row 200: "left" is the sentinel in the max;
+//     the flags still compare it unless the row is band row 200 (only the last row of a column can be);
+//   * steps whose row lies outside the column: no flags, and the pair stores keep H's old half; A's row 0 (band top above
+//     the matrix) is set to 0, which B's first cell reads as its diagonal;
+//   * the first block completes no word of B, a block past lA writes no word of A.
 // 16 bits suffice for the packed differences: every cell of column i is >= -2 i - 209 (the band's top cell reads its left
 // neighbour, which reads its up neighbour; down a column each cell reads its up neighbour) and <= i + 1, so for
-// qlen <= 4000 a difference of two candidates is > -12300.
+// qlen <= 4000 a difference of two candidates is > -12300, and the sentinel plus 2 - x lies in [-24000, -11789].
+constexpr uint32_t SENT2 = 0xB1E0B1E0u;   // -20000 per half: below every cell, so never the maximum and never equal to it
+
+template <bool M> struct Masked { static constexpr bool value = M; };
+
 template <class HS, class SS, class FS, class QF>
 PBSC_DPT_HD void fill_pair(int i, int mlen, int origin, int wbase, HS& H, const SS& S, FS& F, const QF& q, FillBest& best)
 {
@@ -282,159 +331,128 @@ PBSC_DPT_HD void fill_pair(int i, int mlen, int origin, int wbase, HS& H, const 
     const int jbA = origin + i, jbB = jbA + 1;
     const int fA = imax(jbA, 1), fB = imax(jbB, 1);
     const int lA = imin(jbA + BW, nRows) - 1, lB = imin(jbB + BW, nRows) - 1;
+    const int j0 = fA & ~1;
     const int cA = q(i - 1), cB = q(i);
     const uint32_t cArep = (uint32_t)cA * 0x55555u, cBrep = (uint32_t)cB * 0x55555u;
-    // state before step j: column i - 1 at row j - 1 (A's diagonal), A(j - 1), A(j - 2), B(j - 2); row 0 reads 0
-    int hA = H.get(fA - 1), a1 = 0, a2 = 0, b1 = 0;
-    uint32_t wA = 0, wB = 0;
-    int kA = 0, kB = 0, xA = wbase, xB = wbase + W;
-    int vAl = 0, vBl = 0;
-    // the read bases of the single steps, from two 10-base windows in registers (rows x0 + 1 .. x0 + 20): in the passes that
-    // keep the read in global memory a load per step would put its latency on the chain of every step
-    int sx0 = fA - 1;
-    uint32_t sw0 = S.bits(sx0), sw1 = 0;
-    auto sbase = [&](int x)
-    {
-        const int d = x - sx0;
-        return (int)((d < CPW ? sw0 >> (2 * d) : sw1 >> (2 * (d - CPW))) & 3u);
-    };
-    auto step = [&](int j)
-    {
-        int aj = a1;
-        if (j <= lA)
-        {
-            const int left = H.get(j);
-            const int d = hA + (sbase(j - 1) == cA ? 1 : -8);
-            const int l1 = (j == jbA + BW - 1) ? NEVER : left - 1;
-            int v;
-            uint32_t f;
-            if (j == fA)
-            {
-                const int u1 = fA > jbA ? -1 : NEVER;
-                v = imax(d, l1);
-                f = (v == d ? 1u : 0u) | (v == u1 ? 2u : 0u) | (v == l1 ? 4u : 0u);
-                wA = f; kA = (fA & 1) + 1;
-            }
-            else
-            {
-                const int u1 = a1 - 1;
-                v = j == lA ? imax(d, u1) : imax(imax(d, l1), u1);
-                f = (v == d ? 1u : 0u) | (v == u1 ? 2u : 0u) | (v == l1 ? 4u : 0u);
-                wA = (wA << 3) | f;
-                if (++kA == CPW) { F.put(xA++, wA); wA = 0; kA = 0; }
-            }
-            if (j == lA) vAl = v;
-            hA = left; aj = v;
-        }
-        const int r = j - 1;
-        if (r >= fB && r <= lB)
-        {
-            const int d = a2 + (sbase(r - 1) == cB ? 1 : -8);
-            const int l1 = (r == jbB + BW - 1) ? NEVER : a1 - 1;
-            int v;
-            uint32_t f;
-            if (r == fB)
-            {
-                const int u1 = fB > jbB ? -1 : NEVER;
-                v = imax(d, l1);
-                f = (v == d ? 1u : 0u) | (v == u1 ? 2u : 0u) | (v == l1 ? 4u : 0u);
-                wB = f; kB = (fB & 1) + 1;
-            }
-            else
-            {
-                const int u1 = b1 - 1;
-                v = r == lB ? imax(d, u1) : imax(imax(d, l1), u1);
-                f = (v == d ? 1u : 0u) | (v == u1 ? 2u : 0u) | (v == l1 ? 4u : 0u);
-                wB = (wB << 3) | f;
-                if (++kB == CPW) { F.put(xB++, wB); wB = 0; kB = 0; }
-            }
-            H.set(r, v);
-            if (r == lB) vBl = v;
-            b1 = v;
-        }
-        a2 = a1; a1 = aj;
-    };
-    int j = fA;
-    const int jw = (fA & ~1) + CPW;   // first row of A's second flag word
+    pair_sweep(H, fB, lB);
+    // per half, for the masked blocks: "up" of the first cell as its flags see it; the last cell leaves "left" out of the max;
+    // the last cell is band row 200
+    const bool a200 = lA == jbA + BW - 1, b200 = lB == jbB + BW - 1;
+    const uint32_t upF = (jbA <= 0 ? 0u : 0xB1E0u) | (jbB <= 0 ? 0u : 0xB1E00000u);
+    const uint32_t exL = (lA > fA || a200 ? 0xFFFFu : 0u) | (lB > fB || b200 ? 0xFFFF0000u : 0u);
+    const uint32_t row200 = (a200 ? 0xFFFFu : 0u) | (b200 ? 0xFFFF0000u : 0u);
+    // D = (column i - 1 at row j - 1, A(j - 2)): the diagonals; V = (A(j - 1), B(j - 2)): the ups (before j0: no cells)
 #if defined(__CUDA_ARCH__)
-    #pragma unroll 1
-#endif
-    for (; j < jw; j++) step(j);
-    clk_mark(H, CLK_ENDS);
-    // here, at every block: A has no pending flags, B has nine (rows j - 10 .. j - 2)
-#if defined(__CUDA_ARCH__)
-    #pragma unroll 1
-#endif
-    if (j + CPW <= lA)
-    {
-        // D = (column i - 1 at row j - 1, A(j - 2)): the diagonals; V = (A(j - 1), B(j - 2)): the ups
-#if defined(__CUDA_ARCH__)
-        uint32_t D = (uint32_t)(hA & 0xFFFF) | ((uint32_t)a2 << 16), V = (uint32_t)(a1 & 0xFFFF) | ((uint32_t)b1 << 16);
+    uint32_t D = (uint32_t)H.get(j0 - 1) & 0xFFFFu, V = 0u;
 #else
-        uint32_t D = pk16(hA, a2), V = pk16(a1, b1);
+    uint32_t D = pk16(H.get(j0 - 1), 0), V = 0u;
 #endif
-        uint32_t na = S.bits(j - 1), nb = S.bits(j - 2);   // the read windows of the block, loaded one block ahead
+    // the read windows of a block (bases j - 1 .. j + 8 for A, j - 2 .. j + 7 for B), loaded one block ahead; the first one
+    // from the sweep's first base, origin + i - 1 (or 0), shifted: the steps before it compute no cell
+    uint32_t na, nb;
+    {
+        const uint32_t w = S.bits(imax(j0 - 1, 0));
+        na = j0 ? w : w << 2;
+        nb = na << 2;
+    }
+    uint32_t wB = 0, vl = 0;   // B's pending flags (rows j - 10 .. j - 2); (A(lA), B(lB)) once computed
+    int xA = wbase, xB = wbase + W;
+    int j = j0;
+    auto block = [&](auto masked)
+    {
+        constexpr bool M = decltype(masked)::value;
+        // bit s: step s computes a cell of A (row j + s), bit 16 + s: of B (row j + s - 1); the first and the last cells
+        uint32_t inM = 0x03FF03FFu, firstM = 0u, lastM = 0u;
+        bool head = false;
+        if constexpr (M)
+        {
+            auto below = [](int n) { return (1u << imin(imax(n, 0), CPW)) - 1u; };   // steps 0 .. n - 1
+            auto at = [&](int n) { return below(n + 1) & ~below(n); };               // step n
+            inM = (below(lA - j + 1) & ~below(fA - j)) | ((below(lB - j + 2) & ~below(fB - j + 1)) << 16);
+            firstM = at(fA - j) | (at(fB - j + 1) << 16);
+            lastM = at(lA - j) | (at(lB - j + 1) << 16);
+            head = j == j0;
+        }
+        const uint32_t xa = na ^ cArep, xb = nb ^ cBrep;
+        if (!M || j + CPW <= lA) na = S.bits(j + CPW - 1);       // the next block's, when it has cells of A
+        if (!M || j + CPW - 1 <= lB) nb = S.bits(j + CPW - 2);   // ... of B
+        const uint32_t ma = (xa | (xa >> 1)) & 0x55555u, mb = (xb | (xb >> 1)) & 0x55555u;   // bit 2s: step s mismatches
+        const uint32_t m1 = (ma & 0xFFFFu) | (mb << 16);                                       // steps 0..7, both halves
+        const uint32_t m2 = (ma >> 16) | (mb & 0xF0000u);                                      // steps 8, 9
+        uint32_t hw[CPW / 2];
+#if defined(__CUDA_ARCH__)
+        #pragma unroll
+#endif
+        for (int u = 0; u < CPW / 2; u++) hw[u] = H.get2(j + 2 * u, 0);   // each pair on its own: the block may wrap
+        // flags of steps 0..4 and 5..9, per half sum over the steps s of (7 + f_s) * 8^(4 - s mod 5) = 0x7FFF + the three-bit
+        // "equals" flags f_s; at most 14 * 4681 < 2^16, so the halves never carry into each other
+        uint32_t Wa = 0, Wb = 0;
+#if defined(__CUDA_ARCH__)
+        #pragma unroll
+#endif
+        for (int s = 0; s < CPW; s++)
+        {
+            const uint32_t p = (s < 8 ? m1 >> (2 * s) : m2 >> (2 * (s - 8))) & 0x00010001u;
+            const uint32_t e = v2add(D, p * 0xFFF7u + 0x00020002u);   // diagonal + 2 (match) or - 7 per half, no carry across
+            const uint32_t L = prmt(hw[s >> 1], V, (s & 1) ? 0x5432u : 0x5410u);
+            // per half: the step computes its column's first cell, its last cell, a cell at all (constants when unmasked)
+            const uint32_t mf = ((firstM >> s) & 0x00010001u) * 0xFFFFu, ml = ((lastM >> s) & 0x00010001u) * 0xFFFFu;
+            const uint32_t mi = ((inM >> s) & 0x00010001u) * 0xFFFFu;
+            const uint32_t X = v2max3(e, sel16(L, SENT2, ml & exL), sel16(V, SENT2, mf));
+            const uint32_t K = v2add(~X, 0x00030003u);   // 2 - X: max(candidate + K, 1) is 2 where the candidate equals X, else 1
+            uint32_t fU, fL;
+            if constexpr (M)
+            {
+                // the flags' "up" of a first cell and "left" of a last cell are not in the max and may exceed X:
+                // max(min(c + K, X + 2 - c), 1) is 2 where c equals X, else 1
+                const uint32_t X2 = v2add(X, 0x00020002u), U = sel16(V, upF, mf), Lf = sel16(L, SENT2, ml & row200);
+                fU = v2max(v2addmin(U, K, v2sub(X2, U)), 0x00010001u);
+                fL = v2max(v2addmin(Lf, K, v2sub(X2, Lf)), 0x00010001u);
+            }
+            else { fU = v2addmax(V, K, 0x00010001u); fL = v2addmax(L, K, 0x00010001u); }
+            uint32_t f = v2addmax(e, K, 0x00010001u) + (fU << 1) + (fL << 2);
+            f = sel16(0x00070007u, f, mi);   // no flags outside the column
+            if (s < CPW / 2) Wa = (Wa << 3) + f; else Wb = (Wb << 3) + f;
+            uint32_t Vn = v2add(X, 0xFFFFFFFFu);   // X - 1 per half
+            if (M && s == 0 && j == 0) Vn &= 0xFFFF0000u;   // A(0): row 0 reads 0
+            if ((s & 1) == 0)
+            {
+                const uint32_t b2 = prmt(V, Vn, 0x7632u);   // B(j + s - 2), B(j + s - 1)
+                if (s == 0) { if (!head) H.set2(j - 2, 0, b2); }   // inside B's rows in every block but the first
+                else
+                {
+                    const uint32_t t = inM >> (16 + s - 1);   // which of the two rows are B's cells
+                    H.set2(j + s - 2, 0, sel16(hw[s / 2 - 1], b2, ((t & 1u) * 0xFFFFu) | ((t & 2u) * 0x7FFF8000u)));
+                }
+            }
+            vl = sel16(vl, Vn, ml);
+            D = L; V = Vn;
+        }
+        Wa -= 0x7FFF7FFFu; Wb -= 0x7FFF7FFFu;
+        if (!M || j <= lA) F.put(xA++, ((Wa & 0x7FFFu) << 15) | (Wb & 0x7FFFu));
+        if (!head) F.put(xB++, (wB << 3) | (Wa >> 28));
+        wB = ((Wa >> 1) & 0x7FF8000u) | (Wb >> 16);
+        clk_cells(H, M ? CLK_MASKED : CLK_BLOCKS, popc(inM));
+        j += CPW;
+    };
+#if defined(__CUDA_ARCH__)
+    #pragma unroll 1
+#endif
+    do
+    {
+        block(Masked<true>{});   // the first block, then the last one or two
+        clk_mark(H, CLK_MASKED);
 #if defined(__CUDA_ARCH__)
         #pragma unroll 1
 #endif
-        do
-        {
-            const uint32_t xa = na ^ cArep, xb = nb ^ cBrep;
-            if (j + 2 * CPW <= lA) { na = S.bits(j + CPW - 1); nb = S.bits(j + CPW - 2); }
-            const uint32_t ma = (xa | (xa >> 1)) & 0x55555u, mb = (xb | (xb >> 1)) & 0x55555u;   // bit 2s: step s mismatches
-            const uint32_t m1 = (ma & 0xFFFFu) | (mb << 16);                                       // steps 0..7, both halves
-            const uint32_t m2 = (ma >> 16) | (mb & 0xF0000u);                                      // steps 8, 9
-            uint32_t hw[CPW / 2];
-#if defined(__CUDA_ARCH__)
-            #pragma unroll
-#endif
-            for (int u = 0; u < CPW / 2; u++) hw[u] = H.get2(j + 2 * u, 0);   // each pair on its own: the block may wrap
-            // flags of steps 0..4 and 5..9, per half sum over the steps s of (7 + f_s) * 8^(4 - s mod 5) = 0x7FFF + the three-bit
-            // "equals" flags f_s; at most 14 * 4681 < 2^16, so the halves never carry into each other
-            uint32_t Wa = 0, Wb = 0;
-#if defined(__CUDA_ARCH__)
-            #pragma unroll
-#endif
-            for (int s = 0; s < CPW; s++)
-            {
-                const uint32_t p = (s < 8 ? m1 >> (2 * s) : m2 >> (2 * (s - 8))) & 0x00010001u;
-                const uint32_t e = v2add(D, p * 0xFFF7u + 0x00020002u);   // diagonal + 2 (match) or - 7 per half, no carry across
-                const uint32_t L = prmt(hw[s >> 1], V, (s & 1) ? 0x5432u : 0x5410u);
-                const uint32_t X = v2max3(e, L, V);
-                const uint32_t K = v2add(~X, 0x00030003u);   // 2 - X: max(candidate + K, 1) is 2 where the candidate equals X, else 1
-                const uint32_t f = v2addmax(e, K, 0x00010001u) + (v2addmax(V, K, 0x00010001u) << 1) + (v2addmax(L, K, 0x00010001u) << 2);
-                if (s < CPW / 2) Wa = (Wa << 3) + f; else Wb = (Wb << 3) + f;
-                const uint32_t Vn = v2add(X, 0xFFFFFFFFu);   // X - 1 per half
-                if ((s & 1) == 0) H.set2(j + s - 2, 0, prmt(V, Vn, 0x7632u));   // B(j + s - 2), B(j + s - 1)
-                D = L; V = Vn;
-            }
-            Wa -= 0x7FFF7FFFu; Wb -= 0x7FFF7FFFu;
-            F.put(xA++, ((Wa & 0x7FFFu) << 15) | (Wb & 0x7FFFu));
-            F.put(xB++, (wB << 3) | (Wa >> 28));
-            wB = ((Wa >> 1) & 0x7FF8000u) | (Wb >> 16);
-            j += CPW;
-        } while (j + CPW <= lA);
-#if defined(__CUDA_ARCH__)
-        hA = (int)(short)(D & 0xFFFFu); a2 = (int)D >> 16; a1 = (int)(short)(V & 0xFFFFu); b1 = (int)V >> 16;
-#else
-        hA = lo16(D); a2 = hi16(D); a1 = lo16(V); b1 = hi16(V);
-#endif
-        H.set(j - 2, b1);   // the last block left B(j - 2) for the next one
+        while (j + CPW <= lA) block(Masked<false>{});
         clk_mark(H, CLK_BLOCKS);
-    }
-    // the rest reads rows j - 1 .. lA (bases j - 2 .. lA - 1 <= j + 8) and B's last row lB <= lA + 1 (base lB - 1 <= lA)
-    sx0 = j - 2;
-    sw0 = sx0 <= mlen - 1 ? S.bits(sx0) : 0u;
-    sw1 = sx0 + CPW <= imin(lA, mlen - 1) ? S.bits(sx0 + CPW) : 0u;
-#if defined(__CUDA_ARCH__)
-    #pragma unroll 1
-#endif
-    for (; j <= lB + 1; j++) step(j);
-    if (kA) F.put(xA, wA << (3 * (CPW - kA)));
-    if (kB) F.put(xB, wB << (3 * (CPW - kB)));
-    if (lA == nRows - 1) note_last_row(best, vAl, i);
-    if (lB == nRows - 1) note_last_row(best, vBl, i + 1);
-    clk_mark(H, CLK_ENDS);
+    } while (j - 1 <= lB);
+    if (j - 2 <= lB) H.set(j - 2, hi16(V));   // the last block left B(j - 2) for the next one
+    if (j - CPW <= lB) F.put(xB, wB << 3);    // B's last word: rows j - 10 .. j - 2 and no cell in row j - 1
+    if (lA == nRows - 1) note_last_row(best, lo16(vl), i);
+    if (lB == nRows - 1) note_last_row(best, hi16(vl), i + 1);
+    pair_sweep(H, 1, 0);
 }
 
 // Read window.  A sweep from column i (fill_col, or fill_pair of i and i + 1) reads the read from base origin + i - 1 on, and
